@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline measurement of the hot path (contract in the task statement / DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Metric: rollout tokens/s (the reference's actor/output_tokens_per_second, pipelinerl/actor.py:98-106) of the
 sampler's token step on random-init Qwen2.5-7B: 64 running sequences per GPU (actor.llm_max_rollouts,
@@ -57,7 +57,12 @@ def parse():
     ap.add_argument("--no-rollout", action="store_true", help="N = 1: skip the full-rollout run through the plugin API")
     ap.add_argument("--rollout-tokens", type=int, default=8192, help="max_tokens of the full-rollout component")
     ap.add_argument("--splits", default="", help="learner counts of the split runs, e.g. '2,4' (default: by N)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (sampled ids, their logprobs, the logits) as DIR/*.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def workload_config(args, n_gpus):
@@ -131,7 +136,10 @@ def build_engine(args, dev):
     from pipelinerl_b200.model import ModelConfig, ParamArena
     cfg = ModelConfig.qwen2_5_7b(fp32_head=True)   # the reference computes lm_head in fp32 on the sampler
     arena = ParamArena(cfg, dev).init_random(seed=42)
-    room = 256 + args.steps + args.warmup * 2 + 64
+    # every step of the run (warm-up, the launch count, the timed and the end-to-end loops) must fit in max_new_tokens:
+    # a slot that reaches it finishes and stops reading its KV, and the steps after that no longer run the workload
+    steps_run = max(args.warmup, 3) + 1 + 2 * args.steps
+    room = max(256 + args.steps + args.warmup * 2 + 64, steps_run + 1)
     eng = DecodeEngine(cfg, arena, max_batch=args.batch, max_seq_len=args.context + room, max_new_tokens=room,
                        eos_id=-1, seed=42, device=dev, use_cuda_graph=True)
     # synthetic rollout state: every slot has an args.context-token prompt resident in the KV cache
@@ -162,6 +170,26 @@ def algorithmic_bytes(cfg, B, S):
     w_head = (4 if cfg.fp32_head else 2) * cfg.vocab_size * cfg.hidden_size   # hi + lo streams = an fp32 weight's bytes
     kv_per_layer = B * S * 2 * cfg.num_kv_heads * cfg.head_dim * 2
     return w_body + w_head, kv_per_layer
+
+
+DUMP_LOGITS_BYTES = 48 << 20    # the dump stays under 64 MB at any --batch
+
+
+def dump_outputs(out_dir: Path, eng, h_ids, h_lp):
+    """The last end-to-end step's results as float arrays: the sampled ids and logprobs the host received, and the fp32
+    logits they were sampled from (all rows, or a fixed seeded sample of rows when they exceed DUMP_LOGITS_BYTES).
+    The inputs are seeded, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    import torch
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "sampled_ids.npy", h_ids.numpy().astype(np.float64))
+    np.save(out_dir / "sampled_logprobs.npy", h_lp.numpy().astype(np.float32))
+    rows = np.arange(eng.B)
+    max_rows = DUMP_LOGITS_BYTES // (4 * eng.logits.shape[1])
+    if eng.B > max_rows:
+        rows = np.sort(np.random.default_rng(0).choice(eng.B, max_rows, replace=False))
+    np.save(out_dir / "logits_rows.npy", rows.astype(np.float64))
+    np.save(out_dir / "logits.npy", eng.logits.index_select(0, torch.from_numpy(rows).to(eng.logits.device)).cpu().numpy())
 
 
 def run_ours(args):
@@ -229,6 +257,8 @@ def run_ours(args):
         h_tok.copy_(h_ids)
     barrier()
     e2e_ms = (time.perf_counter() - t0) * 1e3
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(Path(args.dump_outputs), eng, h_ids, h_lp)
 
     times = torch.tensor([ms, e2e_ms], dtype=torch.float64, device=dev)
     if world > 1:
