@@ -501,6 +501,23 @@ int prl_sample_logprob(const float* logits /*[B,V]*/, int32_t B, int32_t V, floa
 int prl_sample_logprob_rows(const float* logits /*[B,V]*/, int32_t B, int32_t V, const float* inv_temperature_rows,
                             const uint8_t* greedy_rows, uint64_t seed, uint32_t step, int32_t* out_ids,
                             float* out_logprobs, void* workspace, size_t workspace_bytes, prl_stream_t stream);
+/* top-k / top-p filtering with processed logprobs (vLLM's apply_top_k_top_p + log_softmax of the masked logits).
+ * Call after prl_sample_logprob_rows with the same logits, seed and step.  For every row that is not greedy and has an
+ * active filter (1 <= top_k_rows[b] < V, or top_p_rows[b] < 1) it rewrites out_ids[b] / out_logprobs[b]: the kept set
+ * is {z >= tau}, z = logits[b] * inv_temperature_rows[b], with tau the k-th largest z and then the value where the
+ * softmax mass of the survivors ranked strictly above reaches top_p (every tie with tau is kept); the id is the
+ * Gumbel-max over the kept set with prl_sample_logprob_rows' noise (an unfiltered sample inside the kept set is kept
+ * as is) and the logprob is z[id] - logsumexp(z over the kept set).  Other rows are left untouched.
+ * top_k_rows[b] in {-1, 0} or >= V disables top-k; top_p_rows[b] == 1 disables top-p.  The per-row values live in
+ * device memory, so they are checked on the device: a row with top_p outside (0, 1] or top_k < -1 keeps its
+ * unfiltered sample and reports out_kept[b] = -1.  out_kept[b] (optional) is the kept-set size, V for unfiltered rows.
+ * Deterministic: the same inputs give the same bits. */
+size_t prl_sample_filter_workspace_bytes(int32_t B, int32_t V);
+int prl_sample_filter_rows(const float* logits /*[B,V]*/, int32_t B, int32_t V, const float* inv_temperature_rows,
+                           const uint8_t* greedy_rows, const int32_t* top_k_rows, const float* top_p_rows,
+                           uint64_t seed, uint32_t step, int32_t* out_ids, float* out_logprobs,
+                           int32_t* out_kept /*[B] kept-set size, or NULL*/, void* workspace, size_t workspace_bytes,
+                           prl_stream_t stream);
 /* Device-resident scheduler state of one sampler (all pointers device, one entry per slot).
  * prl_advance_state moves every active slot one token forward without a host round trip:
  * feeds the next prompt token while inside the prompt, else appends (sampled id, logprob) to the

@@ -214,6 +214,10 @@ _SIGNATURES = {
                                       C.c_size_t, C.c_void_p]),
     "prl_sample_logprob_rows": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_uint64,
                                           C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "prl_sample_filter_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
+    "prl_sample_filter_rows": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_size_t, C.c_void_p]),
     "prl_advance_state": (C.c_int, [C.POINTER(EngineState), C.c_void_p]),
     "prl_gemm_bf16_splitk_peer": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int32,
                                             C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -5,7 +5,7 @@ from __future__ import annotations
 from .engine import SamplingParams
 from .llm import LLMCall, LLMOutput, Prompt, TokenLogprob, TrainableLLM
 from .rollouts import TrainingText, apply_rollout_reward
-from .serving import resolve
+from .serving import lookup, resolve
 
 MASKED_TOKEN_ID = -100
 
@@ -34,11 +34,18 @@ def _chat_kwargs(llm: TrainableLLM, prompt: Prompt) -> dict:
     return kw
 
 
-def _reject_unsupported_sampling(params: dict) -> None:
+def _filters_supported(base_url: str) -> bool:
+    """Whether the engine behind `base_url` samples with top-k / top-p (DecodeEngine without the fused head)."""
+    server = lookup(base_url)
+    return bool(getattr(getattr(server, "engine", None), "supports_top_k_top_p", False))
+
+
+def _reject_unsupported_sampling(params: dict, filters_supported: bool) -> None:
     """Sampling features the engine does not implement must fail loudly, exactly as http_shim.py answers 400 for them:
     a silently ignored top_p / top_k / stop would make the recorded logprobs those of a different distribution than the
-    one the request asked for.  (The reference trains with top_p = 1, top_k = -1, no stop strings: conf/base.yaml:46-51.)"""
-    if float(params.get("top_p", 1.0)) < 1.0 or int(params.get("top_k", -1)) > 0:
+    one the request asked for.  (The reference trains with top_p = 1, top_k = -1, no stop strings: conf/base.yaml:46-51;
+    its eval handle samples with top_p 0.95, top_k 50, which engines with `supports_top_k_top_p` serve.)"""
+    if not filters_supported and (float(params.get("top_p") or 1.0) < 1.0 or int(params.get("top_k") or -1) > 0):
         raise ValueError("top_p / top_k sampling is not implemented by this engine")
     if params.get("stop") or params.get("stop_token_ids"):
         raise ValueError("stop strings / stop token ids are not implemented by this engine (eos only)")
@@ -58,11 +65,13 @@ async def llm_async_generate(llm: TrainableLLM, prompt: Prompt, session=None,
     prompt_ids = prompt.token_ids or _token_ids(tok.apply_chat_template(prompt.messages, add_generation_prompt=True,
                                                                         **_chat_kwargs(llm, prompt)))
     params = llm.parameters
-    _reject_unsupported_sampling(params)
+    _reject_unsupported_sampling(params, _filters_supported(llm.base_url))
     max_tokens = int(max_tokens_override if max_tokens_override is not None else params.get("max_tokens", 16))
     temperature = float(params.get("temperature", 1.0))
     sp = SamplingParams(max_tokens=max_tokens, temperature=temperature if temperature > 0 else 1.0,
-                        greedy=temperature <= 0, ignore_eos=bool(params.get("ignore_eos", False)))
+                        greedy=temperature <= 0, ignore_eos=bool(params.get("ignore_eos", False)),
+                        top_k=-1 if params.get("top_k") is None else params["top_k"],
+                        top_p=1.0 if params.get("top_p") is None else params["top_p"])
     req = await resolve(llm.base_url).generate(list(prompt_ids), sp)
     content = tok.decode(req.output_ids)
     call = llm.log_output(prompt, LLMOutput(content=content), count_tokens=False)

@@ -32,6 +32,25 @@ class SamplingParams:
     temperature: float = 1.0
     greedy: bool = False
     ignore_eos: bool = False
+    # vLLM's filters (the reference's eval handle: top_p 0.95, top_k 50): top_k in {-1, 0} or >= vocabulary and
+    # top_p == 1 disable them; greedy requests ignore both.  Logprobs are then those of the filtered, renormalised
+    # distribution (processed_logprobs).
+    top_k: int = -1
+    top_p: float = 1.0
+
+    def __post_init__(self):
+        self.check_filters()
+
+    def check_filters(self) -> None:
+        """The values vLLM accepts (sampling_params.py:_verify_args): top_k an integer >= -1, top_p in (0, 1]."""
+        if isinstance(self.top_k, bool) or not isinstance(self.top_k, int) or self.top_k < -1:
+            raise ValueError(f"top_k must be an integer >= -1 (-1 or 0 disables it), got {self.top_k!r}")
+        if isinstance(self.top_p, bool) or not isinstance(self.top_p, (int, float)) or not 0.0 < self.top_p <= 1.0:
+            raise ValueError(f"top_p must be in (0, 1], got {self.top_p!r}")
+
+    def filtered(self, vocab_size: int) -> bool:
+        """True when top-k or top-p changes this request's distribution."""
+        return not self.greedy and (1 <= self.top_k < vocab_size or self.top_p < 1.0)
 
 
 @dataclass
@@ -47,6 +66,7 @@ class Request:
     model_version: int = 0
     prefilled: int = 0                                   # prompt tokens whose KV is in the cache
     waits_for: list = field(default_factory=list)        # [(request filling a shared page, tokens it must reach)]
+    filtered: bool = False                               # holds its slot's top-k / top-p rows
 
 
 class DecodeEngine:
@@ -124,6 +144,11 @@ class DecodeEngine:
         self.inv_temp_rows = torch.ones(B, dtype=torch.float32, device=d)
         self.greedy_rows = torch.zeros(B, dtype=torch.uint8, device=d)
         self.ignore_eos_rows = torch.zeros(B, dtype=torch.uint8, device=d)
+        # top-k / top-p per slot (-1 / 1.0: off).  The filter kernel runs only while some slot holds a filtered request,
+        # so a batch without one launches exactly the kernels it did before the filters existed.
+        self.top_k_rows = torch.full((B,), -1, dtype=torch.int32, device=d)
+        self.top_p_rows = torch.ones(B, dtype=torch.float32, device=d)
+        self._n_filtered = 0
         self._temperature, self._greedy, self._ignore_eos = 1.0, False, False
         self._graphs: dict[int, torch.cuda.CUDAGraph] = {}
         # ---- chunked prefill + prefix sharing (GRPO attempts share their prompt) ----
@@ -163,6 +188,11 @@ class DecodeEngine:
     def greedy(self, g: bool) -> None:
         self._greedy = bool(g)
         self.greedy_rows.fill_(int(bool(g)))
+
+    @property
+    def supports_top_k_top_p(self) -> bool:
+        """Whether add_request accepts top-k / top-p requests: the fused sampling head has no filter stage."""
+        return not self.fused_head
 
     @property
     def ignore_eos(self) -> bool:
@@ -290,6 +320,13 @@ class DecodeEngine:
                                                self.inv_temp_rows.data_ptr(), self.greedy_rows.data_ptr(), self.seed,
                                                self.step_count, self.sampled.data_ptr(), self.sampled_lp.data_ptr(),
                                                self.sample_ws.data_ptr(), self.sample_ws.numel(), st))
+        if self._n_filtered > 0:
+            # rewrites id / logprob of the filtered slots only; every other slot keeps the sample drawn above
+            _lib.check(lib.prl_sample_filter_rows(self.logits.data_ptr(), self.B, self.cfg.head_rows,
+                                                  self.inv_temp_rows.data_ptr(), self.greedy_rows.data_ptr(),
+                                                  self.top_k_rows.data_ptr(), self.top_p_rows.data_ptr(), self.seed,
+                                                  self.step_count, self.sampled.data_ptr(), self.sampled_lp.data_ptr(),
+                                                  None, None, 0, st))
         _lib.check(lib.prl_advance_state(C.byref(self._state), st))
 
     def step(self) -> None:
@@ -574,6 +611,12 @@ class DecodeEngine:
         self._check_token_ids(prompt_ids)
         if not params.greedy and not params.temperature > 0:
             raise ValueError("temperature must be > 0 (use greedy=True for argmax)")
+        params.check_filters()
+        filtered = params.filtered(self.cfg.vocab_size)
+        if filtered and not self.supports_top_k_top_p:
+            raise ValueError("this engine has no top-k / top-p stage (the fused sampling head and the tensor-parallel "
+                             "engine sample without one): serve top_k / top_p requests from a DecodeEngine built with "
+                             "fused_head=False")
         if self.fused_head and (params.greedy != self._greedy or (not params.greedy and params.temperature != self._temperature)):
             raise ValueError("the fused sampling head takes engine-wide sampling parameters: build the engine with "
                              "fused_head=False to mix requests with different temperature / greedy settings")
@@ -630,6 +673,11 @@ class DecodeEngine:
         self.inv_temp_rows[slot] = 1.0 if params.greedy else 1.0 / float(params.temperature)
         self.greedy_rows[slot] = int(bool(params.greedy))
         self.ignore_eos_rows[slot] = int(bool(params.ignore_eos) or self._ignore_eos)
+        if filtered:
+            req.filtered = True
+            self.top_k_rows[slot] = params.top_k
+            self.top_p_rows[slot] = params.top_p
+            self._n_filtered += 1
         self.tokens[slot] = prompt_ids[start]
         self.positions[slot] = start
         self.seq_lens[slot] = start + 1
@@ -655,6 +703,10 @@ class DecodeEngine:
             req.finish_reason = "stop" if code == 1 else "length"
             self.block_table[slot].zero_()
             self.finished[slot] = 0
+            if req.filtered:
+                self.top_k_rows[slot] = -1
+                self.top_p_rows[slot] = 1.0
+                self._n_filtered -= 1
             self._release_pages(req.pages)
             self.free_slots.append(slot)
             del self.slot_req[slot]

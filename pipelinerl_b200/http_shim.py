@@ -17,8 +17,10 @@ at this shim instead of a vLLM server (SURVEY §8b "wire format"):
   POST /receive_weight_update the reference's trigger for its NCCL broadcast (vllm1.py:244-249).  Here weights arrive by
                               the learner's P2P push; the endpoint only reports the version the sampler is serving.
 
-Sampling features the engine does not implement (top_p < 1, top_k > 0, n > 1, streaming) are rejected with 400 rather
-than silently ignored.  Host code only: the engine behind it is the CUDA DecodeEngine (no CPU fallback).
+Sampling features the engine does not implement (n > 1, streaming; top_p < 1 and top_k > 0 unless the engine has
+`supports_top_k_top_p`) are rejected with 400 rather than silently ignored, and so are top_p / top_k values vLLM would
+reject (top_p outside (0, 1], top_k not an integer >= -1).  Host code only: the engine behind it is the CUDA
+DecodeEngine (no CPU fallback).
 """
 from __future__ import annotations
 
@@ -103,7 +105,13 @@ class HttpShim:
         return web.json_response({"error": {"message": msg, "type": "invalid_request_error"}}, status=400)
 
     def _sampling(self, body: dict) -> SamplingParams | web.Response:
-        if float(body.get("top_p", 1.0)) < 1.0 or int(body.get("top_k", -1)) > 0:
+        top_k = -1 if body.get("top_k") is None else body["top_k"]          # null = vLLM's default
+        top_p = 1.0 if body.get("top_p") is None else body["top_p"]
+        try:
+            filters = SamplingParams(top_k=top_k, top_p=top_p)
+        except ValueError as e:
+            return self._bad(str(e))
+        if (top_p < 1.0 or top_k > 0) and not getattr(self.server.engine, "supports_top_k_top_p", False):
             return self._bad("top_p / top_k sampling is not implemented by this engine (the reference trains with "
                              "top_p=1, top_k=-1, conf/base.yaml:46-51)")
         if int(body.get("n", 1)) != 1 or body.get("stream"):
@@ -111,7 +119,7 @@ class HttpShim:
         temperature = float(body.get("temperature", 1.0))
         max_tokens = int(body.get("max_tokens") or body.get("max_completion_tokens") or self.default_max_tokens)
         return SamplingParams(max_tokens=max_tokens, temperature=temperature if temperature > 0 else 1.0,
-                              greedy=temperature <= 0)
+                              greedy=temperature <= 0, top_k=filters.top_k, top_p=filters.top_p)
 
     async def chat_completions(self, request: web.Request) -> web.Response:
         body = await request.json()

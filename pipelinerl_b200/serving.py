@@ -27,6 +27,13 @@ def resolve(base_url: str) -> "EngineServer":
     return _REGISTRY[name]
 
 
+def lookup(base_url: str) -> "EngineServer | None":
+    """The server registered at `base_url`, or None (unsupported scheme, or nothing registered under that name)."""
+    if not base_url.startswith("inproc://"):
+        return None
+    return _REGISTRY.get(base_url[len("inproc://"):])
+
+
 @dataclass
 class _Pending:
     prompt_ids: list[int]

@@ -153,6 +153,11 @@ class TPDecodeEngine(DecodeEngine):
         s = max(1, min(s, kb_o // 4, kb_d // 4))
         self.split_k["o"] = self.split_k["down"] = s
 
+    @property
+    def supports_top_k_top_p(self) -> bool:
+        """The vocab-parallel head merges sampler partials across ranks; it has no top-k / top-p stage."""
+        return False
+
     def _sample_and_advance(self) -> None:
         lib, st, B, cfg = self.lib, _lib.stream_ptr(), self.B, self.cfg
         group_bytes = B * 16 * 32
